@@ -84,7 +84,37 @@ def parse_args():
     ap.add_argument("--no-comparators", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-baseline-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy, float32 (float64 stays float64), "
+                    "at most 64 MB in all (see dump_outputs)")
     return ap.parse_args()
+
+
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def host_outputs(out) -> dict:
+    """The tensors of a forward's output dict as host numpy arrays: float64 stays float64, everything else becomes float32."""
+    import numpy as np
+
+    return {k: v.detach().cpu().numpy().astype(np.float64 if v.dtype == torch.float64 else np.float32)
+            for k, v in out.items() if isinstance(v, torch.Tensor)}
+
+
+def dump_outputs(arrays: dict, directory: str) -> None:
+    """Write each array as ``<name>.npy`` so that two builds can be compared output for output.  When the arrays exceed
+    DUMP_BUDGET_BYTES together, each is cut to the same share of its elements: a fixed-seed sample of flat positions, in
+    order, so the same arguments always select the same positions."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in sorted(arrays.items()):
+        if total > DUMP_BUDGET_BYTES:
+            flat = a.reshape(-1)
+            keep = np.sort(np.random.default_rng(0).choice(flat.size, flat.size * DUMP_BUDGET_BYTES // total, replace=False))
+            a = flat[keep]
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"outputs of the last timed step written to {directory}: {', '.join(sorted(arrays))}")
 
 
 def load_peaks():
@@ -323,15 +353,18 @@ def run_ours(args):
         pipe = FramePipeline(model, depth=args.inflight, device=dev)
         host_outs = [torch.empty((B, 1, 2, H, W), dtype=dtype).pin_memory() for _ in range(args.inflight)]
 
+    last = {}  # the most recent run_value's last step: its outputs (or, in flight, its pending result) for --dump-outputs
+
     def run_value(n):
         if pipe is None:
             for i in range(n):
-                step_resident(i)
+                last["out"] = step_resident(i)
         else:
             res = [pipe.submit({"images": devin[i % pool]}) for i in range(n)]
             pipe.drain()
             for r in res:
                 r.enqueued()  # re-raises what a slot thread caught: a failed forward must not count as a fast one
+            last["out"] = res[-1]
 
     def run_e2e_any(n):
         if pipe is None:
@@ -396,6 +429,11 @@ def run_ours(args):
             ms_value, _, launches = timed(run_value, args.steps)
             value_remeasured = True
             log(f"resident (re-measured): {ms_value / args.steps:.3f} ms/step")
+        dumped = None
+        if args.dump_outputs and rank == 0:
+            # taken before any later loop calls run_value again: the last timed step always reads devin[(steps - 1) % pool]
+            out = last.pop("out")
+            dumped = host_outputs(out if pipe is None else out.get())
         clocks = sampler.stop()
         log(f"e2e: {ms_e2e / args.steps:.3f} ms/step; clocks {clocks}")
 
@@ -567,6 +605,8 @@ def run_ours(args):
     }
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         result["cpu_baseline"] = cpu_baseline(args, args.cpu_baseline_seconds)
+    if dumped is not None:
+        dump_outputs(dumped, args.dump_outputs)
     if rank == 0:
         print(json.dumps(result), flush=True)
     if world > 1:
@@ -701,8 +741,10 @@ def run_reference(args):
         one_pair()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        one_pair()
+        out = one_pair()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(host_outputs(out), args.dump_outputs)
     value = args.steps / dt
     sample = f"each step = 1 frame pair (of the batch of {args.batch}) at {args.width}x{args.height}, {args.iters} iters, fp32"
     print(json.dumps({

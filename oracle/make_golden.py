@@ -2,7 +2,8 @@
 
 TEST INFRASTRUCTURE (see oracle/__init__.py).  Usage, from the repo root:
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden                          # everything the reference computes on the CPU
+    python -m oracle.make_golden --ref-plugin [--out DIR]  # op_ref_alt_cuda_corr.npz: needs a CUDA device + oracle/_ref
 
 Each fixture stores only the *outputs* of the reference plus a JSON recipe; inputs and
 weights are rebuilt from the recipe with oracle.synth (numpy Philox, platform-stable), so
@@ -11,8 +12,13 @@ the fixtures stay small.  The reference's own tests hold no golden vectors for t
 """
 from __future__ import annotations
 
+import argparse
+import importlib
 import json
 import os
+import sys
+import tempfile
+import types
 
 import numpy as np
 import torch
@@ -36,6 +42,14 @@ E2E_CASES = [
 
 def _recipe(**kw) -> np.ndarray:
     return np.frombuffer(json.dumps(kw, sort_keys=True).encode(), dtype=np.uint8)
+
+
+def _sampled(key: str, t: torch.Tensor, k: int) -> dict:
+    """An output too large to store whole: its shape, the values at synth.sample_index(numel, k), and the sum, absolute
+    sum and largest magnitude over all of it (read back by tests/helpers.check_sample)."""
+    flat = t.detach().double().cpu().reshape(-1).numpy()
+    return {key: flat[synth.sample_index(flat.size, k)].astype(np.float32), key + "_shape": np.array(t.shape),
+            key + "_sums": np.array([flat.sum(), np.abs(flat).sum(), np.abs(flat).max()])}
 
 
 def make_e2e() -> None:
@@ -175,13 +189,94 @@ def make_ops() -> None:
         print("state_shapes", variant, len(shapes), sum(int(np.prod(s)) for k, s in shapes.items() if "running" not in k and "num_batches" not in k))
 
 
+SIBLING_SAME_AS_RAFT = ["gma", "gmflownet", "rapidflow", "rpknet", "skflow", "ms_raft_plus"]
+SIBLING_PER_LEVEL_GEMM = ["sea_raft", "memfof", "flow_anything", "flowseek", "recover"]
+
+
+def make_sibling_corr() -> None:
+    """SURVEY.md section 8(f) rank 3 / appendix E: the CorrBlock of each sibling model's own corr.py, RAFT style
+    (volume + avg-pool pyramid) at two (levels, radius) and SEA-RAFT style (one volume per level) at (3, 3)."""
+    ref_shim.load_raft()
+    b, c, h, w, seed = 2, 32, 17, 24, 61  # 17x24 -> 8x12 -> 4x6 -> 2x3: no 1-pixel level (the reference's sampler divides by W - 1)
+    f1 = torch.from_numpy(synth.synth_normal("sib/f1", (b, c, h, w), seed))
+    f2 = torch.from_numpy(synth.synth_normal("sib/f2", (b, c, h, w), seed))
+    coords = O.coords_grid(b, h, w) + torch.from_numpy(synth.synth_normal("sib/c", (b, 2, h, w), seed, scale=3.0))
+    out = {}
+    for family in SIBLING_SAME_AS_RAFT + SIBLING_PER_LEVEL_GEMM:
+        mod = importlib.import_module(f"ptlflow.models.{family}.corr")
+        with torch.no_grad():
+            if family in SIBLING_SAME_AS_RAFT:
+                for levels, radius in ((4, 4), (2, 3)):
+                    out.update(_sampled(f"{family}_l{levels}_r{radius}", mod.CorrBlock(f1, f2, num_levels=levels, radius=radius)(coords), 1024))
+            else:
+                out.update(_sampled(f"{family}_l3_r3", mod.CorrBlock(f1, f2, 3, 3)(coords), 1024))
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "op_sibling_corr.npz"), recipe=_recipe(b=b, c=c, h=h, w=w, seed=seed), **out)
+    print("op_sibling_corr", len(out) // 3, "outputs")
+
+
+def make_flow_io() -> None:
+    """The reference's .flo writer on a flow holding a NaN, and what its reader returns for the file this project writes."""
+    from ptlflow_b200.utils.flow_utils import flow_write
+
+    ref_shim.load_raft()
+    for absent in ("png", "h5py"):  # pypng / h5py are not in this image; only the .flo branch is exercised
+        sys.modules.setdefault(absent, types.ModuleType(absent))
+    import ptlflow.utils.flow_utils as ref_io
+
+    flow = (np.random.default_rng(4).standard_normal((9, 11, 2)) * 7).astype(np.float32)
+    flow[1, 1] = np.nan
+    with tempfile.TemporaryDirectory() as d:
+        ref_io.flow_write(os.path.join(d, "ref.flo"), flow)
+        flow_write(os.path.join(d, "ours.flo"), flow)
+        written = np.fromfile(os.path.join(d, "ref.flo"), dtype=np.uint8)
+        read = np.asarray(ref_io.flow_read(os.path.join(d, "ours.flo")), dtype=np.float32)
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "io_flo.npz"), recipe=_recipe(h=9, w=11, seed=4, scale=7.0), ref_written=written, ref_read=read)
+    print("io_flo", written.size, "bytes")
+
+
+REF_PLUGIN_CASES = [(1, 256, 16, 24, 16, 24, 4), (2, 128, 17, 29, 8, 14, 4), (1, 64, 9, 12, 9, 12, 3), (1, 256, 55, 128, 27, 64, 4)]
+
+
+def make_ref_plugin(out_dir: str) -> None:
+    """The reference's own native kernel, ``alt_cuda_corr.forward(fmap1, fmap2, coords, radius)`` (oracle/_ref, built by
+    oracle/build_ref.py), on a CUDA device, for the cases of tests/test_gpu_ref_plugin.py."""
+    from . import build_ref
+
+    mod = build_ref.load()
+    if mod is None:
+        raise RuntimeError("oracle/_ref/alt_cuda_corr.so is not built: run oracle/build_ref.py where the reference checkout is")
+    dev = "cuda:0"
+    out = {}
+    for case in REF_PLUGIN_CASES:
+        b, c, h1, w1, h2, w2, r = case
+        f1 = torch.from_numpy(synth.synth_normal("rp/f1", (b, h1, w1, c), 21)).to(dev)
+        f2 = torch.from_numpy(synth.synth_normal("rp/f2", (b, h2, w2, c), 21)).to(dev)
+        grid = torch.stack(torch.meshgrid(torch.arange(w1, dtype=torch.float32), torch.arange(h1, dtype=torch.float32), indexing="xy"), dim=-1)
+        coords = (grid[None, None] * (w2 / w1) + torch.from_numpy(synth.synth_normal("rp/c", (b, 1, h1, w1, 2), 21, scale=3.0))).contiguous().to(dev)
+        (ref,) = mod.forward(f1, f2, coords, r)
+        assert ref.dtype == torch.float32
+        out.update(_sampled("case_" + "_".join(map(str, case)), ref, 4096))
+    os.makedirs(out_dir, exist_ok=True)
+    np.savez_compressed(os.path.join(out_dir, "op_ref_alt_cuda_corr.npz"), recipe=_recipe(seed=21, cases=REF_PLUGIN_CASES), **out)
+    print("op_ref_alt_cuda_corr", len(REF_PLUGIN_CASES), "cases on", torch.cuda.get_device_name(0))
+
+
 def main() -> None:
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--ref-plugin", action="store_true", help="only op_ref_alt_cuda_corr.npz (needs a CUDA device and oracle/_ref)")
+    ap.add_argument("--out", default=GOLDEN_DIR, help="where --ref-plugin writes its fixture")
+    args = ap.parse_args()
+    if args.ref_plugin:
+        make_ref_plugin(args.out)
+        return
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     torch.set_num_threads(max(1, os.cpu_count() or 1))
     make_ops()
     make_e2e()
     make_warm_start()
     make_gma_ops()
+    make_sibling_corr()
+    make_flow_io()
     total = sum(os.path.getsize(os.path.join(GOLDEN_DIR, f)) for f in os.listdir(GOLDEN_DIR))
     print("golden bytes:", total)
 

@@ -94,3 +94,12 @@ def synth_images(batch: int, height: int, width: int, seed: int = 0, kind: str =
 def synth_normal(name: str, shape: Iterable[int], seed: int = 0, scale: float = 1.0) -> np.ndarray:
     """Generic N(0, scale^2) float32 tensor for operator-level fixtures (features, coords noise)."""
     return (scale * _gen(seed, name).standard_normal(tuple(shape), dtype=np.float64)).astype(np.float32)
+
+
+def sample_index(n: int, k: int) -> np.ndarray:
+    """Up to k distinct flat positions spread over [0, n), ascending (all of them when n <= k).  A fixed multiplicative
+    stride rather than an RNG: a fixture that stores a sample of a large output and the test that reads it always agree
+    on the positions."""
+    if n <= k:
+        return np.arange(n)
+    return np.unique((np.arange(k, dtype=np.int64) * 2654435761) % n)

@@ -17,6 +17,19 @@ def load_golden(name):
     return recipe, {k: z[k] for k in z.files if k != "recipe"}
 
 
+def check_sample(mine, g, key, tol):
+    """``mine`` (a whole tensor) against a reference output stored as a sample (oracle/make_golden.py ``_sampled``): same
+    shape, every sampled element within ``tol``, and the sum and absolute sum over all elements within what an
+    element-wise bound of ``tol`` allows."""
+    assert tuple(mine.shape) == tuple(g[key + "_shape"]), (tuple(mine.shape), g[key + "_shape"])
+    flat = mine.detach().double().cpu().reshape(-1).numpy()
+    err = np.abs(flat[synth.sample_index(flat.size, g[key].size)] - g[key]).max()
+    assert err < tol, (key, err)
+    total, abs_total, _ = g[key + "_sums"]
+    assert abs(flat.sum() - total) < tol * flat.size, key
+    assert abs(np.abs(flat).sum() - abs_total) < tol * flat.size, key
+
+
 def e2e_inputs(recipe):
     """(state_dict, images, kwargs) rebuilt from a golden recipe (see oracle/make_golden.py)."""
     kw = dict(recipe["kwargs"])

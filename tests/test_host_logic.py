@@ -225,30 +225,20 @@ def test_flow_io_round_trips_and_conventions(tmp_path):
 
 
 def test_flow_io_agrees_with_reference_reader(tmp_path):
-    """Files written here read back identically through the reference's own flow_read (build container only)."""
-    if not os.path.isdir("/root/reference/ptlflow"):
-        pytest.skip("reference checkout not present")
-    from oracle import ref_shim
+    """Files written here are byte for byte what the reference's own flow_write writes, its flow_read read them back
+    identically, and the reference's file reads back identically here (io_flo.npz, oracle/make_golden.py make_flow_io)."""
+    from helpers import load_golden
     from ptlflow_b200.utils.flow_utils import flow_read, flow_write
 
-    import sys
-    import types
-
-    ref_shim.load_raft()
-    for absent in ("png", "h5py"):  # pypng / h5py are not in this image; only the .flo branch is exercised
-        sys.modules.setdefault(absent, types.ModuleType(absent))
-    try:
-        import ptlflow.utils.flow_utils as ref_io
-    except ImportError as e:
-        pytest.skip(f"reference flow_utils not importable here: {e}")
-
-    flow = (np.random.default_rng(4).standard_normal((9, 11, 2)) * 7).astype(np.float32)
+    recipe, g = load_golden("io_flo")
+    flow = (np.random.default_rng(recipe["seed"]).standard_normal((recipe["h"], recipe["w"], 2)) * recipe["scale"]).astype(np.float32)
     flow[1, 1] = np.nan
     p = tmp_path / "x.flo"
     flow_write(p, flow)
-    ref = ref_io.flow_read(str(p))
+    assert p.read_bytes() == g["ref_written"].tobytes()
+    ref = g["ref_read"]
     assert np.array_equal(np.isnan(ref), np.isnan(flow)) and np.array_equal(ref[~np.isnan(ref)], flow[~np.isnan(flow)])
-    ref_io.flow_write(str(tmp_path / "y.flo"), flow)
+    (tmp_path / "y.flo").write_bytes(g["ref_written"].tobytes())
     mine = flow_read(tmp_path / "y.flo")
     assert np.array_equal(np.isnan(mine), np.isnan(flow)) and np.array_equal(mine[~np.isnan(mine)], flow[~np.isnan(flow)])
 
